@@ -395,6 +395,48 @@ def check_lba_against_oracle(tag, prob, out):
     return float(d)
 
 
+DUMP_STREAMS, DUMP_LBAS = 32, 8    # --dump-outputs sample: a few MB whatever --batch is (the bound is 64 MB)
+
+
+def dump_outputs(out_dir, gb, slabs, match, claimed, nmatch, lba_out):
+    """Writes what the device-resident loop computed in its last timed round as out_dir/<name>.npy (float32 / float64): for a fixed,
+    seeded sample of the streams, the keypoint rows (x, y, size, angle, response, octave, class_id), descriptors, mono counts, match and
+    claimed arrays of SearchByProjection; for a seeded sample of the bundle adjustments, poses, points, per-edge chi2 / depth flags and
+    (iterations, LM trials, lambda, initial chi2, final chi2).  Rows are concatenated over the sampled streams / problems in index order."""
+    import numpy as np
+    B, P = gb[-1][1], len(lba_out)
+    rng = np.random.default_rng(0)
+    streams = np.sort(rng.choice(B, min(B, DUMP_STREAMS), replace=False))
+    probs = np.sort(rng.choice(P, min(P, DUMP_LBAS), replace=False))
+    cols = {k: [] for k in ('keypoints', 'descriptors', 'match', 'claimed')}
+    n_kp, mono, n_match = [], [], []
+    for b in streams:
+        g = next(g for g, (b0, b1) in enumerate(gb) if b0 <= b < b1)
+        i = int(b - gb[g][0])
+        k = int(slabs[g].n[i])
+        kp = slabs[g].kps[i, :k].cpu().numpy()
+        cols['keypoints'].append(np.concatenate([kp[:, :5], kp.view(np.int32)[:, 5:].astype(np.float32)], 1))
+        cols['descriptors'].append(slabs[g].desc[i, :k].cpu().numpy().astype(np.float32))
+        cols['match'].append(match[g][i, :k].cpu().numpy().astype(np.float32))
+        cols['claimed'].append(claimed[g][i, :k].cpu().numpy().astype(np.float32))
+        n_kp.append(k); mono.append(int(slabs[g].mono[i])); n_match.append(int(nmatch[g][i]))
+    out = {'frame_streams': streams.astype(np.float64), 'frame_n_keypoints': np.array(n_kp, np.float64), 'frame_mono': np.array(mono, np.float64),
+           'frame_n_matches': np.array(n_match, np.float64)}
+    out.update({'frame_' + k: np.concatenate(v) for k, v in cols.items()})
+    lba = [lba_out[p] for p in probs]
+    out['lba_problems'] = probs.astype(np.float64)
+    for k in ('poses', 'points', 'chi2'):
+        out['lba_' + k] = np.concatenate([o[k] for o in lba]).astype(np.float64)
+    out['lba_depth_pos'] = np.concatenate([o['depth_pos'] for o in lba]).astype(np.float32)
+    out['lba_stats'] = np.array([[o['iters'], o['trials'], o['lambda_'], o['initial_chi2'], o['final_chi2']] for o in lba], np.float64)
+    total = sum(v.nbytes for v in out.values())
+    if total > 64 << 20:
+        raise SystemExit('--dump-outputs: %d bytes exceed 64 MB' % total)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -410,7 +452,11 @@ def main():
     ap.add_argument('--no-extra', action='store_true', help='skip the BASELINE configs[0] / configs[2] latency lines')
     ap.add_argument('--dev-groups', type=int, default=2, help='stream groups (own handles + CUDA stream) in the device-resident measurement')
     ap.add_argument('--e2e-groups', type=int, default=3, help='stream groups (host threads with their own handles) in flight in the e2e measurement')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the device-resident loop computed in its last timed round (a seeded sample of '
+                    'the streams and bundle adjustments) as DIR/<name>.npy, for comparing two builds output for output')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
         return run_reference(args)
 
@@ -594,6 +640,8 @@ def main():
                                                  g_match[g].cpu().numpy(), g_nmatch[g].cpu().numpy(), L, poses_h[d_last][b0:b1], sf, cam, [0, nb - 1])
     lba_out = opt.download()
     lba_diff = check_lba_against_oracle('device-resident loop', probs[0], lba_out[0])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gb, [g_slab[g][d_last] for g in range(DG)], g_match, g_claimed, g_nmatch, lba_out)
     mean_trials = float(np.mean([o['trials'] for o in lba_out]))
     mean_kp = float(np.mean([float(g_slab[g][d_last].n.float().mean().item()) for g in range(DG)]))
     mean_matches = float(np.mean([float(g_nmatch[g].float().mean().item()) for g in range(DG)]))
@@ -740,7 +788,7 @@ def main():
             run_rounds(0, 2 * LR)
             torch.cuda.synchronize()
             barrier()
-            e2e_steps = max(1, args.steps)
+            e2e_steps = args.steps
             nr = e2e_steps * R
             t0 = time.perf_counter()
             run_rounds(2 * LR, 2 * LR + nr)                         # 2 LR is even: the input sets alternate as in the warm-up

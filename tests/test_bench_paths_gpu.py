@@ -100,6 +100,54 @@ def test_extract_batch_slabs_and_host_batch_matcher(orb, bench, oracle_sets):
         assert np.array_equal(match[b, :k], om) and np.array_equal(claimed[b, :k], oc), b
 
 
+def test_bench_dump_outputs_are_the_timed_loop_results(bench, oracle_sets, tmp_path):
+    """bench.py --dump-outputs at a small size: the dumped keypoints, descriptors and matches of every stream are the oracle's on the
+    frames bench.make_frames rebuilds from their seeds, a dumped bundle adjustment is the oracle's solution of its problem, and the
+    kernel launches the timed loop counted grow in proportion to --steps."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.abspath(bench.__file__))
+    out = str(tmp_path / 'dump')
+    runs = {}
+    for steps in (1, 3):
+        cmd = [sys.executable, os.path.join(root, 'bench.py'), '--steps', str(steps), '--warmup', '1', '--batch', '10', '--rounds', '2', '--lba-rounds', '2',
+               '--no-cpu-baseline', '--no-e2e', '--no-extra'] + (['--dump-outputs', out] if steps == 3 else [])
+        runs[steps] = json.loads(subprocess.check_output(cmd, cwd=root, timeout=900).decode().strip().splitlines()[-1])
+    assert runs[3]['gpu_launches'] == 3 * runs[1]['gpu_launches'] > 0 and runs[3]['config']['frames_per_gpu_per_step'] == 20
+    d = {f[:-4]: np.load(os.path.join(out, f)) for f in os.listdir(out)}
+    assert all(v.dtype in (np.float32, np.float64) for v in d.values()) and sum(v.nbytes for v in d.values()) <= 64 << 20
+    assert np.array_equal(d['frame_streams'], np.arange(10)) and np.array_equal(d['lba_problems'], np.arange(2))
+    from orb_slam3_modified_b200 import synth
+    kl = [oracle_sets[0][1][b][1] for b in range(10)]
+    L = bench.last_frame_slabs(kl, [oracle_sets[0][1][b][2] for b in range(10)], 0, max(len(k) for k in kl))
+    sf = O.OracleExtractor(1000, 1.2, 8, 20, 7).tables()['scale']
+    cam = [float(c) for c in synth.camera(W, H)]
+    o = 0
+    for b in range(10):       # 6 timed rounds: the last one extracted parity 1 and matched it against parity 0
+        omono, okps, odesc = oracle_sets[1][1][b]
+        k, m = len(okps), int(L['nM'][b])
+        assert d['frame_n_keypoints'][b] == k and d['frame_mono'][b] == omono
+        kp = d['frame_keypoints'][o:o + k]
+        assert np.array_equal(kp[:, 0], okps['x']) and np.array_equal(kp[:, 5], okps['octave']) and np.array_equal(d['frame_descriptors'][o:o + k], odesc)
+        last = {n: L[v][b, :m] for n, v in (('valid', 'valid'), ('xyz', 'xyz'), ('octave', 'octave'), ('angle', 'angle'), ('hasObs', 'hasObs'),
+                                            ('descriptors', 'mpDesc'))}
+        om = np.full(k, -1, np.int32); oc = np.zeros(k, np.uint8)
+        on = O.search_last_frame(okps, odesc, (0.0, 0.0, float(W), float(H)), sf, bench.stream_pose(b, 1), cam, last, bench.TH_PROJ, True, om, oc)
+        assert d['frame_n_matches'][b] == on and np.array_equal(d['frame_match'][o:o + k], om) and np.array_equal(d['frame_claimed'][o:o + k], oc)
+        o += k
+    assert o == len(d['frame_keypoints'])
+    # problem 1 (bench's own parity gate checks problem 0): poses / points / statistics are the oracle's solution of that problem
+    nP, nL = bench.LBA_CFG['n_kf'], bench.LBA_CFG['n_pts']
+    prob = bench.lba_problems(2)[1]
+    ref = O.lba_solve(prob)
+    poses, points = d['lba_poses'][nP:2 * nP], d['lba_points'][nL:2 * nL]
+    assert d['lba_poses'].shape == (2 * nP, 7) and d['lba_points'].shape == (2 * nL, 3) and len(d['lba_chi2']) == len(d['lba_depth_pos'])
+    assert d['lba_stats'][1, 0] == ref['iters'] and d['lba_stats'][1, 1] == ref['stats'][3]
+    assert np.abs(O.lba_residuals(prob, poses, points) - O.lba_residuals(prob, ref['poses'], ref['points'])).max() < bench.TOL_PX
+
+
 def test_blurred_planes_equal_oracle(orb, bench):
     """a6: the 7x7 sigma-2 blur of every level, byte for byte (src/ORBextractor.cc:1132-1133)."""
     B = 3
